@@ -19,6 +19,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "oracle")):
@@ -48,7 +49,38 @@ def parse():
     ap.add_argument("--bc-width", default="3x", choices=["1x", "2x", "3x"])
     ap.add_argument("--bc-batch", type=int, default=16)
     ap.add_argument("--bc-steps", type=int, default=4)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+def dump_outputs(path, pd, vpred, ac, state, limit=1 << 20, budget=64 << 20):
+    """Writes the timed forward's results (log-probs, vpred, sampled actions, state out) to path/<name>.npy as float32, so that two
+    builds can be compared output for output.  An array of more than `limit` entries is written as a fixed sample of `limit` of
+    them: the indices come from a generator seeded with the array's name, so every run with the same arguments picks the same ones."""
+    import numpy as np
+
+    arrays = {f"pd_{k}": v for k, v in pd.items()}
+    arrays["vpred"] = vpred
+    arrays.update({f"action_{k}": v for k, v in ac.items()})
+    for i, (mask, (k, v)) in enumerate(state):
+        if mask is not None:
+            arrays[f"state{i}_mask"] = mask
+        arrays[f"state{i}_k"], arrays[f"state{i}_v"] = k, v
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > limit:
+            idx = torch.randint(0, t.numel(), (limit,), generator=torch.Generator().manual_seed(zlib.crc32(name.encode())))
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.float().cpu().numpy()  # integer actions (< 2^24) and masks are exact in float32
+        total += a.nbytes
+        if total > budget:
+            raise RuntimeError(f"--dump-outputs: more than {budget >> 20} MB")
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def peaks():
@@ -518,6 +550,8 @@ def run_ours(args):
     prof, ops.GEMM_PROFILE = ops.GEMM_PROFILE, None
     clocks = sampler.stop() if rank == 0 else None
     nat.device_check()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pd, vpred, ac, state)
     value = world * frames_per_step * args.steps / (ms / 1000.0)
 
     # dominant kernel = gemm_tc_kernel (tcgen05 implicit-GEMM conv + linear): live CUDA-event durations of every launch

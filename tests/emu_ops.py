@@ -40,18 +40,20 @@ def gemm(A, Bw, out, M, N, K, *, conv=None, mr=None, rows_per_group=1, S1=None, 
                  out_scale=out_scale, residual=residual, ld_out=ld, seg=seg if remap else None)
         return out
     Af = A.float()
+    # products summed in fp64 and rounded once to fp32 here and in conv3x3_zp / wgrad: an fp32 sum's order (and with it
+    # which outputs round to the other bf16 neighbour) depends on the host CPU's vector width; this does not
     if conv is not None:
         H, W, Cin = conv
-        x = Af.reshape(-1, H, W, Cin).permute(0, 3, 1, 2)
-        w = Bw.float().reshape(N, 3, 3, Cin).permute(0, 3, 1, 2)
-        acc = F.conv2d(x, w, padding=1).permute(0, 2, 3, 1).reshape(M, N)
+        x = Af.double().reshape(-1, H, W, Cin).permute(0, 3, 1, 2)
+        w = Bw.double().reshape(N, 3, 3, Cin).permute(0, 3, 1, 2)
+        acc = F.conv2d(x, w, padding=1).float().permute(0, 2, 3, 1).reshape(M, N)
         pix = torch.arange(M) % (H * W)
         y, xx = pix // W, pix % W
         cy = torch.where(y == 0, 0, torch.where(y == H - 1, 2, 1))
         cx = torch.where(xx == 0, 0, torch.where(xx == W - 1, 2, 1))
         cls = cy * 3 + cx
     else:
-        acc = Af.reshape(M, K) @ Bw.float().T
+        acc = (Af.double().reshape(M, K) @ Bw.double().T).float()
         cls = torch.zeros(M, dtype=torch.long)
     v = acc
     s1 = S1.reshape(-1, N)[cls] if S1 is not None else 0.0
@@ -123,7 +125,7 @@ def conv3x3_zp(x, Wb, H, W, *, mr=None, S1=None, S2=None, relu=1, residual=None,
         F_, Cin = x.shape[0], x.shape[3]
         Cout = Wb.shape[0]
         xi = from_zp(x).float().permute(0, 3, 1, 2)
-        acc = F.conv2d(xi, Wb.float().reshape(Cout, 3, 3, Cin).permute(0, 3, 1, 2), padding=1).permute(0, 2, 3, 1)  # [F,H,W,Cout]
+        acc = F.conv2d(xi.double(), Wb.double().reshape(Cout, 3, 3, Cin).permute(0, 3, 1, 2), padding=1).float().permute(0, 2, 3, 1)  # [F,H,W,Cout]
         yy, xx = torch.arange(H)[:, None], torch.arange(W)[None, :]
         cls = (torch.where(yy == 0, 0, torch.where(yy == H - 1, 2, 1)) * 3 + torch.where(xx == 0, 0, torch.where(xx == W - 1, 2, 1)))  # [H,W]
         if Ef is not None:
@@ -378,7 +380,7 @@ def wgrad(a, b, shifts=(0,), out=None):
             bs[:R - s] = bf[s:]
         else:
             bs[-s:] = bf[:R + s]
-        cols.append(af.T @ bs)
+        cols.append((af.double().T @ bs.double()).float())
     res = torch.cat(cols, 1)
     if out is not None:
         out.copy_(res)

@@ -1,11 +1,12 @@
 """Caller-side rows f-2 (frame ingest) and f-3 (action codec) + the MineRLAgent mirror.
-CPU: the codec against the live reference (lib/action_mapping.py, lib/actions.py) where /root/reference exists, codec
-properties everywhere, the resize oracle against cv2.  GPU: the resize kernel bit-exact against the oracle / cv2, agent smoke."""
+CPU: the codec against recorded outputs of the reference (lib/action_mapping.py, lib/actions.py), codec
+properties, the resize oracle against cv2.  GPU: the resize kernel bit-exact against the oracle / cv2, agent smoke."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
-import refshim
 import resize_oracle
 import vpt_b200
 from video_pre_training_b200 import agent as A
@@ -23,30 +24,28 @@ def _random_factored(n, rng):
     return dict(buttons=btn, camera=cam)
 
 
-@pytest.mark.skipif(not refshim.available(), reason="/root/reference not present (GPU box)")
 def test_codec_matches_live_reference():
-    import sys
-    ns = refshim.load()
-    import lib.actions as ref_actions  # noqa: E402  (importable once refshim.load() has set up sys.path + stubs)
-    mapper = ns.action_mapping.CameraHierarchicalMapping(n_camera_bins=11)
-    tr = ref_actions.ActionTransformer(**A.ACTION_TRANSFORMER_KWARGS)
+    """The codec against the reference's action mapping and action transformer on the same seeded inputs (outputs recorded by
+    oracle/make_golden.py)."""
+    ref = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference", "codec.npz"))
     codec = A.ActionCodec(**A.ACTION_TRANSFORMER_KWARGS)
-    assert codec.n_buttons_joint == len(mapper.BUTTONS_COMBINATIONS) == 8641
-    assert np.array_equal(codec.idx_to_factored, mapper.BUTTON_IDX_TO_FACTORED)
-    assert np.array_equal(codec.idx_camera_off, mapper.BUTTON_IDX_TO_CAMERA_META_OFF)
+    assert codec.n_buttons_joint == ref["n_combinations"] == 8641
+    assert np.array_equal(codec.idx_to_factored, ref["idx_to_factored"])
+    assert np.array_equal(codec.idx_camera_off, ref["idx_camera_off"])
+
+    def same(out, prefix):
+        keys = sorted(k[len(prefix):] for k in ref.files if k.startswith(prefix))
+        assert sorted(out) == keys and all(np.array_equal(out[k], ref[prefix + k]) for k in keys), prefix
+
     rng = np.random.default_rng(0)
     joint = dict(buttons=rng.integers(0, 8641, (500, 1)), camera=rng.integers(0, 121, (500, 1)))
-    a, b = codec.to_factored(joint), mapper.to_factored({k: v.copy() for k, v in joint.items()})
-    assert np.array_equal(a["buttons"], b["buttons"]) and np.array_equal(a["camera"], b["camera"])
+    same(codec.to_factored(joint), "to_factored.")
     fac = _random_factored(2000, rng)
-    a, b = codec.from_factored(fac), mapper.from_factored({k: v.copy() for k, v in fac.items()})
-    assert np.array_equal(a["buttons"], b["buttons"]) and np.array_equal(a["camera"], b["camera"])
-    e1, e2 = codec.policy2env(fac), tr.policy2env({k: v.copy() for k, v in fac.items()})
-    assert set(e1) == set(e2) and all(np.array_equal(e1[k], e2[k]) for k in e1)
+    same(codec.from_factored(fac), "from_factored.")
+    same(codec.policy2env(fac), "policy2env.")
     env = {"camera": rng.uniform(-15, 15, (300, 2)), "attack": rng.integers(0, 2, 300), "hotbar.3": rng.integers(0, 2, 300)}
-    p1, p2 = codec.env2policy(env), tr.env2policy(env)
-    assert np.array_equal(p1["camera"], p2["camera"]) and np.array_equal(p1["buttons"], p2["buttons"])
-    assert codec.null_buttons_idx == mapper.get_zero_action()["buttons"] and codec.camera_null_idx == mapper.camera_null_idx
+    same(codec.env2policy(env), "env2policy.")
+    assert codec.null_buttons_idx == ref["null_buttons_idx"] and codec.camera_null_idx == ref["camera_null_idx"]
 
 
 def test_codec_properties():

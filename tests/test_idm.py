@@ -1,11 +1,13 @@
 """IDM (BASELINE config 5, SURVEY a19): InverseActionPolicy = conv3d pre-stage + ImpalaCNN (first conv normalised) +
-unmasked transformer + factored heads.  CPU: host logic through the emulated ops vs the oracle (itself bit-exact vs the
-reference, tests/test_oracle.py::test_idm_oracle_matches_live_reference).  GPU: the CUDA path vs the oracle."""
+unmasked transformer + factored heads.  CPU: host logic through the emulated ops vs the oracle (itself pinned to the
+reference, tests/test_idm.py::test_idm_schema_and_oracle_match_live_reference).  GPU: the CUDA path vs the oracle."""
+import os
+
 import pytest
 import torch
 
 import emu_ops
-import refshim
+import make_golden
 import vpt_b200
 import vpt_oracle as O
 from common import perturb
@@ -63,31 +65,22 @@ def test_idm_host_logic_matches_oracle(emulated):
     _compare(pol, sd, cfg, "cpu")
 
 
-@pytest.mark.skipif(not refshim.available(), reason="/root/reference not present (GPU box)")
 def test_idm_schema_and_oracle_match_live_reference():
-    ns = refshim.load()
-    kw = vpt_b200.idm_net_kwargs(impala_width=1, hidsize=64, attention_heads=2, img_shape=[32, 32, 16],
-                                 conv3d_params=dict(inchan=3, outchan=16, kernel_size=[5, 1, 1], padding=[2, 0, 0]), timesteps=8,
-                                 attention_memory_size=8)
-    mapper = ns.action_mapping.IDMActionMapping(n_camera_bins=11)
-    torch.manual_seed(0)
-    ref = ns.policy.InverseActionPolicy(action_space=ns.DictType(**mapper.get_action_space_update()), pi_head_kwargs=dict(temperature=2.0),
-                                        idm_net_kwargs=kw)
-    ref.eval()
-    sd = {k: v.detach().clone() for k, v in ref.state_dict().items()}
+    """The oracle's IDM forward against the reference's, recorded by oracle/make_golden.py on the same weights and frames, and
+    the product's parameter schema against the reference's at a config the CUDA path supports."""
+    rec = torch.load(os.path.join(os.path.dirname(__file__), "golden", "reference", "idm.pt"))
+    kw = rec["idm_net_kwargs"]
+    sd = make_golden.synth_state_dict(rec["weights"])
     cfg = O.Cfg(conv3d=True, **{k: v for k, v in kw.items() if k != "conv3d_params"})
-    img = torch.randint(0, 256, (2, 8, 32, 32, 3), dtype=torch.uint8)
+    img = torch.randint(0, 256, (2, 8, 32, 32, 3), dtype=torch.uint8, generator=torch.Generator().manual_seed(0))
     with torch.no_grad():
-        (pd, _, _), _ = ref(obs={"img": img}, first=torch.zeros(2, 8), state_in=ref.initial_state(2))
         (pd2, _, _), _ = O.idm_policy_forward(sd, cfg, img, torch.zeros(2, 8, dtype=torch.bool), O.initial_state(cfg, 2))
-    assert all(torch.equal(pd[k], pd2[k]) for k in pd)
+    assert set(pd2) == set(rec["pd"])
+    for k in pd2:
+        make_golden.assert_digest(pd2[k], rec["pd"][k], rtol=1e-5, atol=1e-5, what=k)
     # product schema == reference schema at a config the CUDA path supports
-    kw2 = vpt_b200.idm_net_kwargs(**SMALL_IDM)
-    ref2 = ns.policy.InverseActionPolicy(action_space=ns.DictType(**mapper.get_action_space_update()), pi_head_kwargs=dict(temperature=2.0),
-                                         idm_net_kwargs=kw2)
-    ours, _, _ = _make(kw2, pert=False)
-    assert list(ref2.state_dict().keys()) == list(ours.state_dict().keys())
-    assert all(ref2.state_dict()[k].shape == v.shape for k, v in ours.state_dict().items())
+    ours, _, _ = _make(vpt_b200.idm_net_kwargs(**SMALL_IDM), pert=False)
+    assert [(k, tuple(v.shape)) for k, v in ours.state_dict().items()] == rec["schema_small"]
 
 
 @pytest.mark.gpu

@@ -1,12 +1,12 @@
-"""CPU: pins oracle/vpt_oracle.py against (a) fixtures generated from the unmodified reference, (b) the live reference
-when /root/reference is present, (c) the invariants of SURVEY.md section 4."""
+"""CPU: pins oracle/vpt_oracle.py against (a) fixtures generated from the unmodified reference, (b) the reference's own
+outputs recorded under tests/golden/reference/ for the comparisons below, (c) the invariants of SURVEY.md section 4."""
 import glob
 import os
 
 import pytest
 import torch
 
-import refshim
+import make_golden
 import vpt_oracle as O
 
 GOLD = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.pt")))
@@ -40,54 +40,55 @@ def test_golden_fixtures_exist():
     assert len(GOLD) >= 2
 
 
-@pytest.mark.skipif(not refshim.available(), reason="/root/reference not present (GPU box)")
+def _record(name):
+    """What the unmodified reference computed for the comparison, recorded by oracle/make_golden.py."""
+    return torch.load(os.path.join(os.path.dirname(__file__), "golden", "reference", name))
+
+
 @pytest.mark.parametrize("pert", [False, True])
 def test_oracle_matches_live_reference(pert):
-    import make_golden
-
-    pkw = refshim.policy_kwargs("2x", **refshim.TINY)
-    pol = refshim.make_reference_agent_policy(pkw)
-    if pert:
-        make_golden.perturb(pol)
-    sd = {k: v.detach().clone() for k, v in pol.state_dict().items()}
+    """B=3, 5 chunks of uneven length with a reset in the 4th: log-probs, vpred and every layer's state after each chunk, then
+    seeded sampling, against the reference run on the same weights and frames (bit exact on the machine that recorded them)."""
+    rec = _record(f"forward_{'perturbed' if pert else 'plain'}.pt")
+    pkw = rec["policy_kwargs"]
+    sd = make_golden.synth_state_dict(rec["weights"])
     cfg = O.Cfg(**pkw)
-    B = 3
+    B = rec["B"]
     g = torch.Generator().manual_seed(0)
-    st_r, st_o = pol.initial_state(B), O.initial_state(cfg, B)
-    for ci, T in enumerate([8, 8, 3, 8, 1]):
+    st_o = O.initial_state(cfg, B)
+    for ci, (T, ch) in enumerate(zip([8, 8, 3, 8, 1], rec["chunks"])):
         img = torch.randint(0, 256, (B, T, 32, 32, 3), dtype=torch.uint8, generator=g)
         first = torch.zeros(B, T, dtype=torch.bool)
         if ci == 3:
             first[1, 0] = True
         with torch.no_grad():
-            (pd, v, _), st_r = pol({"img": img}, first, st_r)
             (pd2, v2, _), st_o = O.agent_policy_forward(sd, cfg, img, first, st_o)
-        for k in pd:
-            assert torch.equal(pd[k], pd2[k])
-        assert torch.equal(v, v2)
-        for a, b in zip(st_r, st_o):
-            assert torch.equal(a[0], b[0]) and torch.equal(a[1][0], b[1][0]) and torch.equal(a[1][1], b[1][1])
-    torch.manual_seed(7)
-    a1 = pol.pi_head.sample(pd)
+        for k in pd2:
+            make_golden.assert_digest(pd2[k], ch["pd"][k], rtol=1e-5, atol=1e-5, what=(ci, k))
+        make_golden.assert_digest(v2, ch["v"], rtol=1e-5, atol=1e-5, what=(ci, "vpred"))
+        for (m, dk, dv), (m2, (k2, v2_)) in zip(ch["state"], st_o):
+            assert torch.equal(m, m2)
+            make_golden.assert_digest(k2, dk, rtol=1e-5, atol=1e-6, what=(ci, "K"))
+            make_golden.assert_digest(v2_, dv, rtol=1e-5, atol=1e-6, what=(ci, "V"))
     torch.manual_seed(7)
     a2 = O.sample(pd2)
-    assert all(torch.equal(a1[k], a2[k]) for k in a1)
-    assert torch.equal(pol.pi_head.logprob(a1, pd), O.logprob(pd2, a2))
+    assert all(torch.equal(rec["sample"][k], a2[k]) for k in a2)
+    assert torch.allclose(rec["logprob"], O.logprob(pd2, a2), rtol=1e-5, atol=1e-5)
 
 
-@pytest.mark.skipif(not refshim.available(), reason="/root/reference not present (GPU box)")
 def test_oracle_matches_live_reference_128px():
     """One full-size 128x128 frame through the 1x-width CNN path with reduced transformer (config C1 shape)."""
-    pkw = refshim.policy_kwargs("1x", n_recurrence_layers=1)
-    pol = refshim.make_reference_agent_policy(pkw)
-    sd = {k: v.detach().clone() for k, v in pol.state_dict().items()}
+    rec = _record("forward_128px.pt")
+    pkw = rec["policy_kwargs"]
+    sd = make_golden.synth_state_dict(rec["weights"])
     cfg = O.Cfg(**pkw)
     img = torch.randint(0, 256, (1, 1, 128, 128, 3), dtype=torch.uint8, generator=torch.Generator().manual_seed(3))
     first = torch.zeros(1, 1, dtype=torch.bool)
     with torch.no_grad():
-        (pd, v, _), _ = pol({"img": img}, first, pol.initial_state(1))
         (pd2, v2, _), _ = O.agent_policy_forward(sd, cfg, img, first, O.initial_state(cfg, 1))
-    assert torch.equal(pd["buttons"], pd2["buttons"]) and torch.equal(pd["camera"], pd2["camera"]) and torch.equal(v, v2)
+    for k in ("buttons", "camera"):
+        make_golden.assert_digest(pd2[k], rec["pd"][k], rtol=1e-5, atol=1e-5, what=k)
+    make_golden.assert_digest(v2, rec["v"], rtol=1e-5, atol=1e-5, what="vpred")
 
 
 def _tiny():
@@ -130,43 +131,35 @@ def test_flop_model_matches_survey():
         assert abs(O.forward_flops_per_frame(O.Cfg(**O.widths(w))) / 1e9 - gf) < 1e-3
 
 
-@pytest.mark.skipif(not refshim.available(), reason="/root/reference not present (GPU box)")
 def test_oracle_gradient_matches_live_reference_autograd():
     """The BC step's parity target is autograd through the oracle (tests/test_training.py); this pins that target itself: the
     gradient of the BC loss (behavioural_cloning.py:101-123: -log-prob of the demonstrated action, KV memory detached between
     chunks) through the unmodified reference equals the gradient through the oracle, parameter by parameter."""
-    import make_golden
-
-    pkw = refshim.policy_kwargs("2x", **refshim.TINY)
-    pol = refshim.make_reference_agent_policy(pkw)
-    make_golden.perturb(pol)
-    pol.train()  # as behavioural_cloning.py leaves it (no dropout / batch-norm in these models: same function)
-    sd = {k: v.detach().clone() for k, v in pol.state_dict().items()}
+    rec = _record("gradient.pt")
+    pkw = rec["policy_kwargs"]
+    sd = make_golden.synth_state_dict(rec["weights"])
     cfg = O.Cfg(**pkw)
     B, T = 2, 8
     g = torch.Generator().manual_seed(3)
-    st_r, st_o = pol.initial_state(B), O.initial_state(cfg, B)
-    for ci in range(2):
+    st_o = O.initial_state(cfg, B)
+    for ch in rec["chunks"]:
         img = torch.randint(0, 256, (B, T, 32, 32, 3), dtype=torch.uint8, generator=g)
         first = torch.zeros(B, T, dtype=torch.bool)
         actions = {"camera": torch.randint(0, 121, (B, T, 1), generator=g), "buttons": torch.randint(0, 8641, (B, T, 1), generator=g)}
-        for p in pol.parameters():
-            p.grad = None
-        (pd, _, _), st_r = pol({"img": img}, first, st_r)
-        loss_r = -pol.pi_head.logprob(actions, pd).mean()
-        loss_r.backward()
-        st_r = [(m, (k.detach(), v.detach())) for (m, (k, v)) in st_r]  # tree_map(lambda x: x.detach(), ...) :111
         leaf = {k: v.clone().requires_grad_(v.dtype.is_floating_point) for k, v in sd.items()}
         (pd_o, _, _), st_o = O.agent_policy_forward(leaf, cfg, img, first, st_o)
         loss_o = -O.logprob(pd_o, actions).mean()
         loss_o.backward()
         st_o = [(m, (k.detach(), v.detach())) for (m, (k, v)) in st_o]
-        assert torch.equal(loss_r.detach(), loss_o.detach())
+        assert torch.allclose(ch["loss"], loss_o.detach(), rtol=1e-6, atol=0)
         n_checked = 0
-        for name, p in pol.named_parameters():
-            if p.grad is None:
+        for name, d in ch["grads"].items():
+            if d is None:
                 assert leaf[name].grad is None, name  # value head: untouched by the BC loss in both
                 continue
-            assert torch.allclose(p.grad, leaf[name].grad, rtol=1e-5, atol=1e-8), name
+            # a recorded gradient comes from another machine, where fp32 sums run in another order: entries far below the
+            # parameter's largest one carry that rounding, so the absolute slack is 1e-5 of the largest recorded entry
+            scale = (d["full"] if "full" in d else d["sample"]).abs().max().item()
+            make_golden.assert_digest(leaf[name].grad, d, rtol=1e-5, atol=1e-5 * scale, what=name)
             n_checked += 1
         assert n_checked > 80
