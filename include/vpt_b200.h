@@ -386,6 +386,19 @@ int vpt_attention_bwd(const void* Q, const void* Kf, const void* Vf, const float
  *                                                                                          lib/action_head.py:176-184 */
 int vpt_softmax_bwd(const float* logp, const int64_t* idx, float scale, void* out, int64_t ld_out, int32_t col0, int64_t rows, int32_t n,
                     void* stream);
+/* Loss and gradient of the RL fine-tuning step (training.RLTrainer), one CTA per frame row.  Per head h (nheads <= 4): student
+ * log-softmax logp[h] fp32 [rows][n[h]], teacher logp_teacher[h] (logp_teacher == NULL: no teacher, KL term and statistic 0), taken
+ * action idx[h] [rows], gradient columns col0[h] of dlog.  Per row: old_logp, adv, ret, vpred fp32 [rows]; mu_rsig fp32 [2] on the
+ * device = (mean, 1/std) of the return normaliser.  With lp = sum_h logp[h][a_h], ratio = exp(lp - old_logp), tn = (ret - mean)/std:
+ *   dlog[r][col0[h] + j] = inv_temp * (g [j == a_h] + q_j (kl_coef*inv_n (pd_j - pd_t,j - kl_h) + ent_coef*inv_n (pd_j + H_h) - g))  (bf16)
+ *   dlog[r][col_v]       = 2 vf_coef inv_n (vpred - tn)                                                                         (bf16)
+ * where g = -ratio*adv*inv_n, or 0 where the clipped surrogate is the minimum (ratio > 1+clip_eps with adv > 0, ratio < 1-clip_eps
+ * with adv < 0).  stats fp32 [rows][5] = (lp, sum_h kl_h, sum_h H_h, (vpred - tn)^2, clipped flag).
+ *                                           lib/action_head.py:176-220, lib/scaled_mse_head.py:37-43, lib/normalize_ewma.py:26-35 */
+int vpt_rl_heads_bwd(const float* const* logp, const float* const* logp_teacher, const int64_t* const* idx, const int32_t* n,
+                     const int32_t* col0, int32_t nheads, const float* old_logp, const float* adv, const float* ret, const float* vpred,
+                     const float* mu_rsig, float clip_eps, float kl_coef, float ent_coef, float vf_coef, float inv_temp, float inv_n,
+                     void* dlog, int64_t ld_out, int32_t col_v, float* stats, int64_t rows, void* stream);
 
 #ifdef __cplusplus
 }

@@ -13,7 +13,7 @@ from .types import DictType, Discrete, TensorType, idm_action_space, minecraft_a
 from .agent import ActionCodec, IDMAgent, MineRLAgent, composite_cursor, ingest_frames, resize_frames  # noqa: F401
 from .policy import InverseActionNet, InverseActionPolicy, MinecraftAgentPolicy, MinecraftPolicy, NetConfig  # noqa: F401
 from .checkpoint import load_model_parameters, load_training_state, load_weights, save_training_state, save_weights  # noqa: F401
-from .training import BCTrainer  # noqa: F401
+from .training import BCTrainer, RLTrainer  # noqa: F401
 from .parallel import FlatAdamDP  # noqa: F401
 
 POLICY_KWARGS_2X = dict(  # agent.py:16-36

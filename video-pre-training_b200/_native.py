@@ -137,6 +137,9 @@ SIGNATURES = {
     "vpt_firstconv_bwd_parts": (_I, [_L, _I, _I]),
     "vpt_attention_bwd": (_I, [_P, _P, _P, _P, _L, _P, _P, _L, _P, _P, _P, _L, _P, _P, _I, _I, _I, _I, _I, _P]),
     "vpt_softmax_bwd": (_I, [_P, _P, _F, _P, _L, _I, _L, _I, _P]),
+    # RL step (training.RLTrainer)
+    "vpt_rl_heads_bwd": (_I, [C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_I), C.POINTER(_I), _I, _P, _P, _P, _P, _P, _F, _F, _F, _F,
+                              _F, _F, _P, _L, _I, _P, _L, _P]),
 }
 
 _lib = None

@@ -34,6 +34,7 @@ void set_error(const char* fmt, ...) {
 #include "firstconv_bwd.cuh"
 #include "precise.cuh"
 #include "codec.cuh"
+#include "rl_heads.cuh"
 
 extern "C" const char* vpt_last_error(void) { return vpt::g_err; }
 extern "C" int vpt_abi_version(void) { return VPT_ABI_VERSION; }

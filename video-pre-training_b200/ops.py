@@ -533,3 +533,7 @@ def codec_from_env(buttons, camera, thresholds, nbins, strides, inventory_idx):
               "vpt_codec_from_env")
     _count()
     return out
+
+
+# ---- RL fine-tuning step (csrc/rl_heads.cuh; training.RLTrainer) --------------------------------------------------------
+from .rl_ops import rl_heads_bwd  # noqa: E402,F401

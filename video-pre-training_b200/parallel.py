@@ -80,7 +80,9 @@ class FlatAdamDP:
     torch.optim.Adam semantics with L2 weight decay; 1/world_size folded into the kernel).
 
     Pass only the parameters that receive a gradient (behavioural cloning: everything but `value_head.*`, whose `.grad` stays None in
-    the reference): torch.optim.Adam SKIPS a parameter without a gradient (no weight decay, no moment update), whereas a slice of this
+    the reference; the RL step, training.RLTrainer: every parameter with requires_grad, `value_head.linear.*` included -- the return
+    normaliser's buffers are requires_grad=False and stay out of the bucket): torch.optim.Adam SKIPS a parameter without a gradient
+    (no weight decay, no moment update), whereas a slice of this
     bucket that is never written would still be decayed.  `step()` therefore refuses parameters whose `.grad` no longer aliases the
     bucket (e.g. after `zero_grad(set_to_none=True)` on the module) instead of silently applying Adam to zeros."""
 

@@ -679,8 +679,8 @@ class _PolicyBase(nn.Module):
             self._hpprep_fp = fp
         return self._hpprep
 
-    def _heads_fp(self):
-        return tuple((p.data_ptr(), p._version) for n, p in self.named_parameters() if not n.startswith("net."))
+    def _heads_fp(self):  # (the return normaliser is not part of the heads' kernel-side weights)
+        return tuple((p.data_ptr(), p._version) for n, p in self.named_parameters() if not n.startswith(("net.", "value_head.normalizer.")))
 
     def _build_heads_prepared(self):
         ws, bs, cols, c0 = [], [], OrderedDict(), 0

@@ -16,8 +16,12 @@ What each layer type needs (u = gamma * n + beta is the normalised layer input, 
 
 The KV memory carried in `state_in` is detached exactly like behavioural_cloning.py:111 (`tree_map(lambda x: x.detach())`),
 and `value_head.*` receives no gradient (None in the reference: the BC loss never touches it).
+
+`RLTrainer` shares the taped forward, the backward and the weight re-layout; only its loss block differs (clipped policy gradient,
+KL to a frozen teacher, entropy, value loss -- one kernel, csrc/rl_heads.cuh), and it also trains `value_head.linear.*`.
 """
 import torch
+import torch.distributed as dist
 
 from . import ops
 from .policy import BF16, F32, MinecraftAgentPolicy
@@ -36,6 +40,11 @@ def _tr(W, pad_to=None):
     return Wt.contiguous()
 
 
+def _relayout_fp(policy):
+    """Fingerprint of the parameters the weight re-layout reads: not the return normaliser, which every RL step updates."""
+    return tuple((p.data_ptr(), p._version) for n, p in policy.named_parameters() if not n.startswith("value_head.normalizer."))
+
+
 def _acc(p, g):
     """p.grad += g (allocating on first use), like autograd's accumulation."""
     g = g.reshape(p.shape)
@@ -47,6 +56,8 @@ def _acc(p, g):
 
 class BCTrainer:
     """`loss, state_out = trainer.loss_and_grad(img, first, state_in, actions)` accumulates d loss / d param into `.grad`."""
+
+    value_column = False  # RLTrainer: the value head rides in column ntot of the heads' dgrad / wgrad GEMMs
 
     def __init__(self, policy: MinecraftAgentPolicy):
         if not isinstance(policy, MinecraftAgentPolicy):
@@ -70,7 +81,7 @@ class BCTrainer:
 
     # -- backward-side weight layouts (re-made whenever a parameter changes, like policy._Prepared) -------------------
     def _weights(self):
-        fp = tuple((p.data_ptr(), p._version) for p in self.policy.parameters())
+        fp = _relayout_fp(self.policy)
         if self._wprep is not None and fp == self._wprep_fp:
             return self._wprep
         with torch.no_grad():
@@ -86,7 +97,7 @@ class BCTrainer:
         pol, net = self.policy, self.policy.net
         from .policy import _Prepared, _fingerprint
         fp_net, fp_heads = _fingerprint(net), pol._heads_fp()
-        fp_all = tuple((p.data_ptr(), p._version) for p in pol.parameters())
+        fp_all = _relayout_fp(pol)
         if net._prep is not None and net._prep_fp == fp_net and pol._hprep is not None and pol._hprep_fp == fp_heads and self._wprep is not None \
                 and self._wprep_fp == fp_all:
             return
@@ -147,9 +158,12 @@ class BCTrainer:
                                     mlp1_t=_tr(P[f"{b}.mlp1.layer.weight"])))
         w["last_t"] = _tr(P["lastlayer.layer.weight"])
         self.ntot = sum(getattr(pol.pi_head, name).linear_layer.weight.shape[0] for name in pol.head_specs)
-        self.ld_logits = (self.ntot + 7) // 8 * 8
-        cat = torch.cat([getattr(pol.pi_head, name).linear_layer.weight for name in pol.head_specs], 0)
-        w["heads_t"] = _tr(cat, self.ld_logits)
+        rows = [getattr(pol.pi_head, name).linear_layer.weight for name in pol.head_specs]
+        if self.value_column:  # value weight as row ntot: dlat, its wgrad row and col_sums column come out of the heads' GEMMs
+            rows.append(pol.value_head.linear.weight)
+        self.ld_logits = (len(rows) - len(pol.head_specs) + self.ntot + 7) // 8 * 8
+        assert not self.value_column or self.ntot < self.ld_logits
+        w["heads_t"] = _tr(torch.cat(rows, 0), self.ld_logits)
         return w
 
     # -- generic pieces -------------------------------------------------------------------------------------------------
@@ -215,6 +229,29 @@ class BCTrainer:
     def loss_and_grad(self, img, first, state_in, actions, upper_grads_ready=None):
         """`upper_grads_ready()` is called once every gradient except those of `img_process.cnn.stacks.*` is final (the ImpalaCNN
         backward, most of the step's time, is still to come): the hook for `FlatAdamDP.reduce_async`."""
+        return self._step(img, first, state_in, lambda pd, vpred, N: self._nll_dlog(pd, actions, N), upper_grads_ready)
+
+    def _nll_dlog(self, pd, actions, N):
+        """BC loss block: -mean joint log-prob of the taken actions -> (d loss / d head GEMM outputs, loss)."""
+        pol = self.policy
+        hp = pol._heads_prepared()
+        dlog = torch.zeros((N, self.ld_logits), dtype=BF16, device=pd[next(iter(pd))].device)
+        scale = 1.0 / (pol.temperature * N)
+        logp = None
+        for name, (shape, n) in pol.head_specs.items():
+            c0, width = hp["cols"][name]
+            if width != n:
+                raise NotImplementedError("BCTrainer: heads with several sub-actions are not trained by the reference")
+            idx = actions[name].reshape(N).to(torch.int64)
+            lp = ops.gather_logprob(pd[name].reshape(N, n), idx)
+            logp = lp if logp is None else logp + lp
+            ops.softmax_bwd(pd[name].reshape(N, n), idx, scale, dlog, c0)
+        loss = -logp.sum() / N
+        return dlog, loss
+
+    def _step(self, img, first, state_in, loss_block, upper_grads_ready):
+        """Taped forward, `loss_block(pd, vpred, N) -> (dlog, result)` (d loss / d head GEMM outputs, bf16 [N][ld_logits]), then the
+        hand-written backward from dlog to every parameter gradient.  Returns (result, state_out)."""
         pol, net = self.policy, self.policy.net
         cfg = net.cfg
         self.refresh_weights()
@@ -232,30 +269,24 @@ class BCTrainer:
         finally:
             net._tape = None
         if self.keep_tape:
+            tape["latent"] = lat_bf16
             self.last_tape = tape
-        pd, _ = pol._heads(lat_bf16, B, t)
+        pd, vpred = pol._heads(lat_bf16, B, t)
         # ---------------- loss + d logits ----------------
+        dlog, result = loss_block(pd, vpred, N)
         hp = pol._heads_prepared()
-        dlog = torch.zeros((N, self.ld_logits), dtype=BF16, device=img.device)
-        scale = 1.0 / (pol.temperature * N)
-        logp = None
-        for name, (shape, n) in pol.head_specs.items():
-            c0, width = hp["cols"][name]
-            if width != n:
-                raise NotImplementedError("BCTrainer: heads with several sub-actions are not trained by the reference")
-            idx = actions[name].reshape(N).to(torch.int64)
-            lp = ops.gather_logprob(pd[name].reshape(N, n), idx)
-            logp = lp if logp is None else logp + lp
-            ops.softmax_bwd(pd[name].reshape(N, n), idx, scale, dlog, c0)
-        loss = -logp.sum() / N
         # ---------------- heads ----------------
-        dWh = ops.wgrad(dlog, lat_bf16)[: self.ntot]
+        nrow = self.ntot + (1 if self.value_column else 0)
+        dWh = ops.wgrad(dlog, lat_bf16)[:nrow]
         dbh = ops.col_sums(dlog)[1]
         for name in pol.head_specs:
             c0, width = hp["cols"][name]
             lin = getattr(pol.pi_head, name).linear_layer
             _acc(lin.weight, dWh[c0:c0 + width])
             _acc(lin.bias, dbh[c0:c0 + width])
+        if self.value_column:
+            _acc(pol.value_head.linear.weight, dWh[self.ntot:nrow])
+            _acc(pol.value_head.linear.bias, dbh[self.ntot:nrow])
         dlat = self._gemm(dlog, wts["heads_t"], h)
         self._dbg("latent", dlat)
         del dlog
@@ -277,7 +308,7 @@ class BCTrainer:
             upper_grads_ready()
         # ---------------- ImpalaCNN, last stack to first ----------------
         self._cnn_bwd(dcnn, tape, wts, P)
-        return loss, state_out
+        return result, state_out
 
     def _dense_bwd(self, dz, tape, wts, P):
         cfg = self.policy.net.cfg
@@ -385,3 +416,116 @@ class BCTrainer:
                 dx = self._normconv_bwd(dfull, rec["x_in"], rec["mr_in"], rec["H_in"], rec["W_in"], wts["stacks"][i]["first"],
                                         f"{s}.firstconv", P)
                 del dfull
+
+
+class RLTrainer(BCTrainer):
+    """RL fine-tuning step of `MinecraftAgentPolicy`: clipped policy gradient, KL to a frozen pretrained teacher, entropy bonus and
+    the value head's loss in normalised space (lib/action_head.py:176-220, lib/scaled_mse_head.py:37-43, lib/normalize_ewma.py:26-55).
+
+        stats, state_out, teacher_state_out = tr.loss_and_grad(img, first, state_in, teacher_state_in, actions,
+                                                               old_logp, advantages, returns, upper_grads_ready=None)
+
+    One call covers N = B*T frames.  Per frame i: the taken action a_i (one index per head), old_logp_i (the joint log-prob recorded at
+    rollout), the advantage A_i and the return R_i, all computed by the caller.  pd is the student's per-head log-softmax of the
+    logits divided by the temperature (what `forward` returns), pd_t the teacher's, q = exp(pd):
+
+        lp_i  = sum_h pd_h[i, a_h,i]                                          (joint, as `logprob`)
+        r_i   = exp(lp_i - old_logp_i)
+        pg_i  = -min(r_i A_i, clip(r_i, 1 - clip_eps, 1 + clip_eps) A_i)
+        kl_i  = sum_h sum_j q_h,j (pd_h,j - pd_t,h,j)                          (= get_kl_of_action_dists(pd, pd_teacher): student first)
+        ent_i = sum_h -sum_j q_h,j pd_h,j
+        tn_i  = (R_i - mu) / sigma    with (mu, sigma^2) = running_mean_var() AFTER this batch's EWMA update (norm_axes = 2)
+        loss  = mean_i pg_i + kl_coef mean_i kl_i - ent_coef mean_i ent_i + vf_coef mean_i (vpred_i - tn_i)^2
+
+    vpred is the raw (normalised-space) value output.  Gradients wrt the temperature-scaled logits z of head h (times 1/temperature
+    for the GEMM output): g_i (delta_ja - q_j) with g_i = -r_i A_i / N, or 0 where the clipped term is the minimum (r > 1 + clip_eps
+    with A > 0, r < 1 - clip_eps with A < 0); (kl_coef/N) q_j ((pd_j - pd_t,j) - kl_h,i); (ent_coef/N) q_j (pd_j + H_h,i); and
+    d/dvpred_i = 2 vf_coef (vpred_i - tn_i) / N.  All of it is one kernel (ops.rl_heads_bwd).  The value head sits in column ntot
+    of the heads' gradient buffer, so its backward rides in the heads' dgrad / wgrad / bias-sum launches.
+
+    The return normaliser (`value_head.normalizer.*`) is updated in place by every call with the batch mean and mean square of R,
+    averaged over the ranks of an initialised torch.distributed group (one all-reduce of two floats), so every replica holds the
+    normaliser a single process would hold for the global batch.  No step synchronises with the host.  The teacher (a frozen
+    `MinecraftAgentPolicy` with the same heads) runs its bf16 inference forward on the same frames with its own KV memory; its
+    parameters are never written.  `stats` holds 0-d device tensors: loss, pg, kl, entropy, value, clipfrac (the fraction of frames
+    whose clipped term is the minimum, i.e. that pass no policy gradient).  bf16 only; heads with several sub-actions are refused."""
+
+    value_column = True
+    norm_beta = 0.99999  # NormalizeEwma defaults (lib/normalize_ewma.py:9): beta, epsilon, per_element_update=False
+    norm_eps = 1e-5
+
+    def __init__(self, policy: MinecraftAgentPolicy, teacher=None, *, clip_eps=0.2, kl_coef=0.0, ent_coef=0.0, vf_coef=1.0):
+        super().__init__(policy)
+        if policy.net.precision != "bf16":
+            raise NotImplementedError("RLTrainer: bf16 precision only")
+        if teacher is not None:
+            if not isinstance(teacher, MinecraftAgentPolicy):
+                raise TypeError("RLTrainer: the teacher is a MinecraftAgentPolicy")
+            if teacher is policy:
+                raise ValueError("RLTrainer: the teacher must be a separate, frozen policy (e.g. a copy of the pretrained weights)")
+            if dict(teacher.head_specs) != dict(policy.head_specs):
+                raise ValueError("RLTrainer: the teacher's action heads differ from the student's")
+            if teacher.net.precision != "bf16":
+                raise NotImplementedError("RLTrainer: bf16 precision only (teacher)")
+        if kl_coef != 0 and teacher is None:
+            raise ValueError("RLTrainer: kl_coef != 0 needs a teacher")
+        self.teacher = teacher
+        self.clip_eps, self.kl_coef, self.ent_coef, self.vf_coef = float(clip_eps), float(kl_coef), float(ent_coef), float(vf_coef)
+
+    def _update_normalizer(self, returns):
+        """EWMA update of value_head.normalizer with this batch (lib/normalize_ewma.py:37-52) -> fp32 [2] (mean, 1/std) after it."""
+        nz = self.policy.value_head.normalizer
+        R = returns.reshape(-1)
+        mom = torch.stack([R.mean(), (R * R).mean()])
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            dist.all_reduce(mom, op=dist.ReduceOp.SUM)  # equal shards: the mean of the rank means is the global batch mean
+            mom = mom / dist.get_world_size()
+        w = self.norm_beta
+        with torch.no_grad():
+            nz.running_mean.mul_(w).add_(mom[0:1] * (1.0 - w))
+            nz.running_mean_sq.mul_(w).add_(mom[1:2] * (1.0 - w))
+            nz.debiasing_term.mul_(w).add_(1.0 * (1.0 - w))
+            deb = nz.debiasing_term.clamp(min=self.norm_eps)
+            mean = nz.running_mean / deb
+            var = (nz.running_mean_sq / deb - mean ** 2).clamp(min=1e-2)
+            return torch.cat([mean, torch.rsqrt(var)]).to(F32).contiguous()
+
+    def loss_and_grad(self, img, first, state_in, teacher_state_in, actions, old_logp, advantages, returns, upper_grads_ready=None):
+        """`upper_grads_ready()`: as in BCTrainer.loss_and_grad (the value head's gradient is final by then)."""
+        B, t = img.shape[:2]
+        N = B * t
+        for name, x in (("old_logp", old_logp), ("advantages", advantages), ("returns", returns)):
+            if tuple(x.shape) != (B, t) or x.dtype != F32 or x.device != img.device:
+                raise ValueError(f"RLTrainer: {name} must be a float32 ({B}, {t}) tensor on {img.device}, got {x.dtype} {tuple(x.shape)} on {x.device}")
+        pd_t, teacher_state_out = None, None
+        if self.teacher is not None:
+            with torch.no_grad():
+                (pd_t, _, _), st = self.teacher({"img": img}, first, teacher_state_in)
+            teacher_state_out = [(m, (k.detach(), v.detach())) for (m, (k, v)) in st]
+        mu_rsig = self._update_normalizer(returns)
+        old, adv, ret = old_logp.reshape(N).contiguous(), advantages.reshape(N).contiguous(), returns.reshape(N).contiguous()
+
+        def loss_block(pd, vpred, n_rows):
+            pol = self.policy
+            hp = pol._heads_prepared()
+            dlog = torch.zeros((N, self.ld_logits), dtype=BF16, device=img.device)
+            lps, lts, idx, cols = [], [], [], []
+            for name, (shape, n) in pol.head_specs.items():
+                c0, width = hp["cols"][name]
+                if width != n:
+                    raise NotImplementedError("RLTrainer: heads with several sub-actions are not trained")
+                lps.append(pd[name].reshape(N, n))
+                if pd_t is not None:
+                    lts.append(pd_t[name].reshape(N, n))
+                idx.append(actions[name].reshape(N).to(torch.int64).contiguous())
+                cols.append(c0)
+            rs = ops.rl_heads_bwd(lps, lts if pd_t is not None else None, idx, cols, old, adv, ret, vpred.reshape(N).contiguous(), mu_rsig,
+                                  self.clip_eps, self.kl_coef, self.ent_coef, self.vf_coef, 1.0 / pol.temperature, 1.0 / N, dlog, self.ntot)
+            m = rs.mean(0)  # (lp, kl, entropy, value loss, clipped)
+            r = torch.exp(rs[:, 0] - old)
+            pg = -torch.minimum(r * adv, r.clamp(1.0 - self.clip_eps, 1.0 + self.clip_eps) * adv).mean()
+            loss = pg + self.kl_coef * m[1] - self.ent_coef * m[2] + self.vf_coef * m[3]
+            return dlog, dict(loss=loss, pg=pg, kl=m[1], entropy=m[2], value=m[3], clipfrac=m[4])
+
+        stats, state_out = self._step(img, first, state_in, loss_block, upper_grads_ready)
+        return stats, state_out, teacher_state_out
